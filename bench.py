@@ -9,7 +9,7 @@ geometric verification (two_view_geometry.cc:292-489) -- the reference's SiftFea
 candidate list.  `value` = candidate pairs verified per second with the images resident in HBM; `e2e` = the same pass
 with descriptors, keypoints and pairs coming from pinned host memory and results + match / inlier lists going back.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]
     python bench.py --impl reference ...     # the reference's CPU path (oracle port) on the host cores
 
 Multi-GPU: ONE pair list, cut into contiguous (locality-ordered) ranges, one per rank; rank 0 gathers the results
@@ -70,7 +70,32 @@ def parse():
                     help="pairs per b2_match_pairs_device -> b2_verify_pairs_device call (one launch group of the stage kernels)")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the C3 results of the last step as DIR/<name>.npy (float64; a fixed, "
+                         f"seeded sample of {DUMP_MAX_PAIRS} pairs when there are more) to compare two builds output for output")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "b200":
+        ap.error("--dump-outputs writes the results of the b200 arm")
+    return a
+
+
+DUMP_MAX_PAIRS = 1 << 17      # 38 float64 values per pair: at most 40 MB in all
+
+
+def dump_outputs(out_dir, results, pairs):
+    """What a caller of the timed C3 step receives -- one RESULT_DTYPE row per candidate pair -- as one float64 .npy per
+    field, with the pairs and their indices in the candidate list.  The inputs are seeded, so the same arguments give the
+    same files on any build that computes the same thing."""
+    n = len(results)
+    idx = np.arange(n) if n <= DUMP_MAX_PAIRS else np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_PAIRS, replace=False))
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    np.save(d / "pair_index.npy", idx.astype(np.float64))
+    np.save(d / "pairs.npy", pairs[idx].astype(np.float64))
+    for f in results.dtype.names:
+        np.save(d / f"{f}.npy", results[f][idx].astype(np.float64))
 
 
 # --------------------------------------------------------------------- workload
@@ -549,6 +574,7 @@ def bench_pipeline(a, dev, local_rank, rank, world, cores, barrier, dist):
     ev1.record()
     barrier()
     wall = time.perf_counter() - wall0
+    last_step = gathered
     launches = lib().b2_kernel_launch_count() - launches0
     clocks = sampler.stop()
     if world > 1:
@@ -564,7 +590,7 @@ def bench_pipeline(a, dev, local_rank, rank, world, cores, barrier, dist):
         hd = host.numpy()
         hdescs = [hd[i] for i in range(a.seq_images)]
         kps = list(coll["keypoints"])
-        e_steps = max(1, min(a.steps, 2))
+        e_steps = a.steps
         d2h = 0
         t_setup = t_run = 0.0
 
@@ -605,7 +631,7 @@ def bench_pipeline(a, dev, local_rank, rank, world, cores, barrier, dist):
         out["results"] = {"config_histogram": {int(k): int(c) for k, c in zip(*np.unique(g["config"], return_counts=True))},
                           "mean_inliers_of_verified": float(g["n_inliers"][g["config"] > 1].mean()) if (g["config"] > 1).any() else 0.0,
                           "trials_per_pair": {k: float(g[k + "_num_trials"].mean()) for k in ("E", "F", "H")}}
-        out["_gathered"] = g
+        out["_gathered"], out["_last_step"] = g, last_step
     out["_coll"], out["_pairs"], out["_seeds"], out["_fm"] = coll, pairs_all, seeds_all, fm
     return out
 
@@ -622,13 +648,13 @@ def bench_retrieval_sharded(a, coll, local_rank, rank, world, barrier, dist, pai
     g = VocabSimilarityGraph(box[0], num_images=2 * a.seq_cand, num_nearest_neighbors=5, device=local_rank)
     walls = []
     pairs = None
-    for s in range(1 + 2):
+    for s in range(a.warmup + a.steps):
         barrier()
         t0 = time.perf_counter()
         pairs, _sc = g.RunSharded(coll["desc"], rank, world, dist)
         barrier()
         walls.append(time.perf_counter() - t0)
-    w = float(np.mean(walls[1:]))
+    w = float(np.mean(walls[a.warmup:]))
     t = torch.tensor([g.timing.get("word_search_s", 0.0), g.timing.get("index_build_s", 0.0), g.timing.get("query_s", 0.0)],
                      dtype=torch.float64, device=coll["desc"].device)
     dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -661,13 +687,13 @@ def bench_retrieval(a, coll, local_rank, cores, pairs_all):
     try:
         vi.set_vocabulary(vocab)
         steps = []
-        for s in range(1 + 2):
+        for s in range(a.warmup + a.steps):
             torch.cuda.synchronize()
             t0 = time.perf_counter()
             vi.index_images_device(coll["desc"].data_ptr(), n_img, n_kp, K)
             ids, sc, cnt = vi.query_all(n_ret)
             w = time.perf_counter() - t0
-            if s >= 1:
+            if s >= a.warmup:
                 steps.append((w, vi.last_timing()))
         w = float(np.mean([x[0] for x in steps]))
         tm = {k: float(np.mean([x[1][k] for x in steps])) for k in steps[0][1]}
@@ -725,7 +751,7 @@ def bench_match(a, dev, local_rank, rank, world, barrier, dist):
     cap = max(64 << 20, int(n_pairs) * 64)
     off_dev = torch.empty(n_pairs + 1, dtype=torch.int64, device=dev)
     mat_dev = torch.empty((cap, 2), dtype=torch.int32, device=dev)
-    steps, warm = max(1, min(a.steps, 2)), max(1, min(a.warmup, 2))
+    steps, warm = a.steps, a.warmup
     for _ in range(warm):
         m.match_pairs_device(n_pairs, pairs_dev.data_ptr(), opt, off_dev.data_ptr(), mat_dev.data_ptr(), cap)
     barrier()
@@ -862,6 +888,9 @@ def main():
     fm = pl.pop("_fm")
     coll, pairs_all, seeds_all = pl.pop("_coll"), pl.pop("_pairs"), pl.pop("_seeds")
     gathered = pl.pop("_gathered", None)
+    last_step = pl.pop("_last_step", None)
+    if rank == 0 and a.dump_outputs:
+        dump_outputs(a.dump_outputs, last_step, pairs_all)
 
     # ------------------------------------------------------------------ CPU baseline + parity spot check (rank 0)
     cpu = None

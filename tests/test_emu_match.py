@@ -33,7 +33,9 @@ def mm():
             raise RuntimeError(f"emulated library error {rc}: {L2.b2_last_error().decode()}")
     mt.check = check
     yield mt
-    lm._lib, lm.LIB_PATH, mt.check = None, real_path, saved[1]
+    # the product library object comes back itself: the wrapper modules bound their argtypes on it once (a fresh CDLL
+    # would leave e.g. bundle_adjustment's raw-pointer arguments unconverted, truncated to C ints)
+    lm._lib, lm.LIB_PATH, mt.check = saved[0], real_path, saved[1]
 
 
 def test_reference_cpu_vs_gpu_cases(mm):

@@ -2,6 +2,8 @@
 (src/retrieval/visual_index_test.cc:84-112: an indexed image queried with its own descriptors ranks first with a
 strictly larger score, result sizes follow max_num_images) and against a plain numpy restatement of the scoring formula
 (idf weights, Hamming weights, burstiness and the two normalisations)."""
+from pathlib import Path
+
 import numpy as np
 
 from dagsfm_b200.retrieval import make_vocabulary
@@ -100,19 +102,28 @@ def test_exact_word_search_equals_the_references_flann_golden_vectors():
         assert (d2 == g[f"dist_k{k}"].astype(np.int64)).all()
 
 
-def test_exact_word_search_equals_the_vendored_flann_live_where_it_is_built():
-    """The same comparison against oracle/_ref/libflann_ref.so itself (present wherever `make -C oracle ref` ran with the
-    reference tree, and on the GPU box, where the prebuilt file travels) on fresh random cases."""
-    import pytest
-    if not orc.flann_ref_available():
-        pytest.skip("oracle/_ref/libflann_ref.so not built")
+def flann_random_cases():
+    """Random vocabularies (one word duplicated where there are more than 20) and descriptor sets: (words, desc, k) per case."""
     rng = np.random.default_rng(7)
     for n_words, n, k in ((33, 100, 5), (700, 400, 5), (1, 10, 1), (129, 64, 8)):
         words = rng.integers(0, 256, (n_words, 128)).astype(np.uint8)
         if n_words > 20:
             words[n_words // 2] = words[3]
         desc = rng.integers(0, 256, (n, 128)).astype(np.uint8)
-        o = orc.RetrievalOracle(words, np.zeros((64, 128), np.float32), np.zeros((n_words, 64), np.float32), np.ones(n_words, np.uint8))
-        kk = min(k, n_words)
-        ids, _ = orc.flann_ref_knn_linear(words, desc, kk)
-        assert (o.word_ids(desc, kk) == ids).all()
+        yield words, desc, min(k, n_words)
+
+
+def flann_case_digest(words, desc, k):
+    import hashlib
+    return hashlib.sha256(words.tobytes() + desc.tobytes() + bytes([k])).hexdigest()
+
+
+def test_exact_word_search_equals_the_vendored_flann_on_random_cases():
+    """The same comparison on random cases: tests/golden/retrieval_flann_random.npz holds the nearest words the reference's
+    vendored FLANN (oracle/_ref/libflann_ref.so, exact mode) returned for flann_random_cases(), with a digest of each case's
+    inputs; generator tests/golden/make_retrieval_flann_golden.py."""
+    g = np.load(Path(__file__).parent / "golden" / "retrieval_flann_random.npz")
+    for i, (words, desc, k) in enumerate(flann_random_cases()):
+        assert str(g[f"digest_{i}"]) == flann_case_digest(words, desc, k), f"case {i}: inputs differ from the stored ones"
+        o = orc.RetrievalOracle(words, np.zeros((64, 128), np.float32), np.zeros((len(words), 64), np.float32), np.ones(len(words), np.uint8))
+        assert (o.word_ids(desc, k) == g[f"ids_{i}"]).all()
